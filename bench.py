@@ -60,7 +60,31 @@ def parse():
     ap.add_argument("--no-lib-baseline", action="store_true", help="skip the reference-generator-on-cuDNN side leg")
     ap.add_argument("--no-png", action="store_true", help="skip the e2e pass that also writes the PNG files")
     ap.add_argument("--no-strong", action="store_true", help="N>1: skip the strong-scaling pass (one clip split over ranks)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32/float64, <= 64 MB in all), "
+                         "so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
+
+
+DUMP_BUDGET = 64 * 10 ** 6 - 2 ** 16       # bytes of .npy files --dump-outputs may write (room left for the headers)
+
+
+def dump_frames(out_dir, frames_d):
+    """uint8 BGR frames (T,S,S,3) of the last timed step -> out_dir/frames.npy (float32, codes 0..255) and
+    out_dir/frame_ids.npy (float64 clip indices).  A clip larger than the budget is cut to a fixed seeded sample of
+    whole frames, the same sample for the same arguments."""
+    import numpy as np
+    import torch
+    T = frames_d.shape[0]
+    n = max(1, min(T, (DUMP_BUDGET - 8 * T) // (frames_d[0].numel() * 4)))
+    ids = np.arange(T) if n == T else np.sort(np.random.Generator(np.random.PCG64(0)).choice(T, n, replace=False))
+    frames = frames_d[torch.as_tensor(ids, device=frames_d.device)].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frames.npy"), frames)
+    np.save(os.path.join(out_dir, "frame_ids.npy"), ids.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -306,6 +330,10 @@ def run_train(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:     # the losses the last timed step returned, one float64 scalar per term
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(args.dump_outputs, "loss_%s.npy" % k), np.asarray(float(v), dtype=np.float64))
     if world > 1:
         t = torch.tensor([ms], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t)
     clocks = sampler.stop() if sampler else None
@@ -451,6 +479,8 @@ def main():
     launches0 = _lib.launch_count()
     ms, wall = timed(step_device, args.steps, sampler)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:     # out_d holds every frame of the last timed step (rank 0's clip)
+        dump_frames(args.dump_outputs, out_d)
     fps = world * T * args.steps / (ms * 1e-3)
     for _ in range(1):
         step_e2e()

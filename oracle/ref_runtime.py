@@ -1,8 +1,7 @@
 """Run the REFERENCE's own classes (TEST INFRASTRUCTURE ONLY, see oracle/__init__.py).
 
-Imports ``iPERCore`` from the staged tree ``oracle/_ref`` (oracle/build_ref.py; falls back to /root/reference in the build
-container) and builds the real ``iPERCore.models.imitator.Imitator`` on synthetic assets, because the real ones are not
-available offline (SURVEY.md §8c):
+Imports ``iPERCore`` from the staged tree ``oracle/_ref`` (oracle/build_ref.py) and builds the real
+``iPERCore.models.imitator.Imitator`` on synthetic assets, because the real ones are not available offline (SURVEY.md §8c):
 
 * ``neural_renderer`` (third-party CUDA extension, absent): a stub module with upstream's ``look_at`` /
   ``vertices_to_faces`` (plain torch) and ``rasterize_face_index_map_and_weight_map`` backed by oracle/raster_ref.c on the
@@ -29,10 +28,9 @@ STAGED = os.path.join(HERE, "_ref")
 
 
 def ref_root():
-    for root in (STAGED, "/root/reference"):
-        if os.path.isdir(os.path.join(root, "iPERCore")):
-            return root
-    raise FileNotFoundError("the reference tree is not staged: run oracle/build_ref.py where /root/reference exists")
+    if os.path.isdir(os.path.join(STAGED, "iPERCore")):
+        return STAGED
+    raise FileNotFoundError("the reference tree is not staged under oracle/_ref: run oracle/build_ref.py")
 
 
 def available():

@@ -40,14 +40,15 @@ def main():
     out_dir = os.path.join(a.work, "patched" if a.patched else "stock")
     os.makedirs(out_dir, exist_ok=True)
     im = rr.build_imitator(opt, a.device)
+    sync = torch.cuda.synchronize if a.device.startswith("cuda") else (lambda: None)
     src_smpl, tgt = rr.synthetic_clip(model, a.frames, ns=a.ns)
     paths = rr.write_source_images(a.work, a.ns, a.size)
     t0 = time.time()
     info = im.source_setup(paths, src_smpl, masks=None, bg_img=None, offsets=0, links_ids=None)
-    torch.cuda.synchronize()
+    sync()
     t1 = time.time()
     outs = im.inference(tgt, cam_strategy="smooth", output_dir=out_dir, prefix="pred_", verbose=False)
-    torch.cuda.synchronize()
+    sync()
     t2 = time.time()
     np.savez_compressed(os.path.join(out_dir, "source.npz"), uv_img=info["uv_img"].float().cpu().numpy(),
                         bg=info["bg"].float().cpu().numpy(), f2pts=info["f2pts"].float().cpu().numpy(),

@@ -111,14 +111,20 @@ def test_weight_packing_layouts():
     assert heads.w.shape == (2, 32, 320) and float(heads.w[:, 20:].abs().max()) == 0.0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/iPERCore"), reason="reference tree only exists in the build container")
+def _staged_reference():
+    from oracle import ref_runtime as rr
+    return rr.ref_root() if rr.available() else None
+
+
+@pytest.mark.skipif(_staged_reference() is None, reason="reference tree not staged (oracle/build_ref.py)")
 def test_patch_install_against_reference():
     """install() wires the seams into the REAL iPERCore package (import level; runs in a subprocess to keep sys.modules clean)."""
     import subprocess
     import sys
+    ref = _staged_reference()
     code = r"""
 import sys, types
-sys.path.insert(0, %r); sys.path.insert(0, "/root/reference")
+sys.path.insert(0, %r); sys.path.insert(0, %r)
 import numpy as np; np.int = int; np.float = float
 ed = types.ModuleType("easydict")
 class AD(dict):
@@ -129,7 +135,7 @@ import ipercore_b200.patch as p
 p.install()
 import toml
 from iPERCore.models.networks import NetworksFactory
-cfg = AD(toml.load("/root/reference/assets/configs/neural_renders/AttLWB-SPADE.toml")["Generator"])
+cfg = AD(toml.load(%r)["Generator"])
 g = NetworksFactory.get_by_name("AttLWB-SPADE", cfg=cfg, temporal=False)
 assert type(g).__module__ == "ipercore_b200.generator" and len(g.state_dict()) == 221
 from iPERCore.models import imitator as imod
@@ -139,7 +145,7 @@ assert imod.Imitator.inference.__module__ == "ipercore_b200.patch"
 import neural_renderer
 assert neural_renderer.__name__ == "ipercore_b200.neural_renderer"
 print("OK")
-""" % ROOT
+""" % (ROOT, ref, os.path.join(ref, "assets", "configs", "neural_renders", "AttLWB-SPADE.toml"))
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0 and "OK" in out.stdout, out.stderr[-2000:]
 

@@ -1,6 +1,7 @@
 """Context measurement (not a parity test): the plain PyTorch/cuDNN formulation of the per-frame path on the same B200 —
 "the existing Blackwell kernel to beat" of SURVEY.md §8d / BASELINE.md §3 — using the oracle's torch-functional
-restatement moved to cuda:0.  Writes gpurun_out/torch_gpu_baseline.json; asserts only sanity."""
+restatement moved to cuda:0.  Prints the rates (and writes them to torch_gpu_baseline.json in the test's temporary
+directory); asserts only sanity."""
 import json
 import os
 import time
@@ -15,7 +16,7 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("S", [512])
-def test_pytorch_cudnn_path_timing(S, template):
+def test_pytorch_cudnn_path_timing(S, template, tmp_path):
     import make_golden
     dev = "cuda:0"
     sd = {k: v.to(dev) for k, v in weights.synth_state_dict(0).items()}
@@ -41,6 +42,5 @@ def test_pytorch_cudnn_path_timing(S, template):
                 res["%s_bs%d_fps" % (name, bs)] = n * bs / (time.perf_counter() - t0)
     torch.backends.cudnn.allow_tf32 = True
     print("PyTorch/cuDNN forward_tsf %dx%d on %s:" % (S, S, torch.cuda.get_device_name(0)), json.dumps(res))
-    os.makedirs("gpurun_out", exist_ok=True)
-    json.dump(res, open("gpurun_out/torch_gpu_baseline.json", "w"), indent=1)
+    json.dump(res, open(os.path.join(tmp_path, "torch_gpu_baseline.json"), "w"), indent=1)
     assert all(v > 0 for v in res.values())
