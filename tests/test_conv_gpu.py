@@ -63,16 +63,47 @@ def _expected(x, wp, conv, P):
     return y
 
 
-@pytest.mark.parametrize("P", [2, 1, 3])
-@pytest.mark.parametrize("N,H,W,Cin,Cout,mode,k", CASES)
-def test_conv_gemm_planes(N, H, W, Cin, Cout, mode, k, P):
+def _unpack(m, Cin, Cout, mode, k):
+    """packed (rows_total, K) -> the reference's weight layout"""
+    if mode == 2:
+        kidx = {0: (1, 3), 1: (0, 2)}
+        wt = torch.zeros(Cin, Cout, 4, 4)
+        for py in range(2):
+            for px in range(2):
+                blk = m[(py * 2 + px) * Cout:(py * 2 + px + 1) * Cout]
+                for ta in range(2):
+                    for tb in range(2):
+                        wt[:, :, kidx[py][ta], kidx[px][tb]] = blk[:, (ta * 2 + tb) * Cin:(ta * 2 + tb + 1) * Cin].t()
+        return wt
+    return m.reshape(Cout, k, k, Cin).permute(0, 3, 1, 2).contiguous()
+
+
+def _planes_problem(N, H, W, Cin, Cout, mode, k, P):
+    """seeded operands of a CASES row and the fp32 reference of the rounded operands: (x, w, bias, exp, atol, rtol)"""
     from ipercore_b200 import ops
-    from ipercore_b200.ops import Planes
     x = _rand((N, Cin, H, W), 1)
     wshape = (Cin, Cout, 4, 4) if mode == 2 else (Cout, Cin, k, k)
     fan = Cin * (4 if mode == 2 else k * k)
     w = _rand(wshape, 2, scale=(3.0 / fan) ** 0.5)
     bias = _rand((Cout,), 3, 0.1)
+    wp = (ops.pack_convT_weight if mode == 2 else ops.pack_conv_weight)(w, P)
+
+    class _W:
+        def effective(self_inner):
+            return tuple(None if t is None else _unpack(t, Cin, Cout, mode, k) for t in wp.effective())
+    exp = F.relu(_expected(x, _W(), lambda xx, ww: _ref_conv(xx, ww, mode, k), P) + bias.view(1, -1, 1, 1))
+    # remaining differences: fp32 accumulation order over K (<= 3456 terms), the dropped lo*lo term (P=2), and the
+    # precision of the OUTPUT planes themselves (P=1: 11 bits; P=3: ~15 bits; P=2: ~22 bits)
+    atol, rtol = {2: (1e-4, 0), 3: (1.5e-4, 1e-4), 1: (5e-4, 1.1e-3)}[P]
+    return x, w, bias, exp, atol, rtol
+
+
+@pytest.mark.parametrize("P", [2, 1, 3])
+@pytest.mark.parametrize("N,H,W,Cin,Cout,mode,k", CASES)
+def test_conv_gemm_planes(N, H, W, Cin, Cout, mode, k, P):
+    from ipercore_b200 import ops
+    from ipercore_b200.ops import Planes
+    x, w, bias, exp, atol, rtol = _planes_problem(N, H, W, Cin, Cout, mode, k, P)
     a = Planes.from_nchw(x.to(DEV), P)
     wp = (ops.pack_convT_weight if mode == 2 else ops.pack_conv_weight)(w, P).to(DEV)
     oH, oW = (H // 2, W // 2) if mode == 1 else ((2 * H, 2 * W) if mode == 2 else (H, W))
@@ -81,28 +112,8 @@ def test_conv_gemm_planes(N, H, W, Cin, Cout, mode, k, P):
     ops.conv_gemm(a, wp, mode, k, rows, 256 if rows >= 256 else rows, ops.IPER_EPI_PLANES, bias=bias.to(DEV), relu=True,
                   out=out)
     torch.cuda.synchronize()
-
-    def unpack(m):      # packed (rows_total, K) -> the reference's weight layout
-        if mode == 2:
-            kidx = {0: (1, 3), 1: (0, 2)}
-            wt = torch.zeros(Cin, Cout, 4, 4)
-            for py in range(2):
-                for px in range(2):
-                    blk = m[(py * 2 + px) * Cout:(py * 2 + px + 1) * Cout]
-                    for ta in range(2):
-                        for tb in range(2):
-                            wt[:, :, kidx[py][ta], kidx[px][tb]] = blk[:, (ta * 2 + tb) * Cin:(ta * 2 + tb + 1) * Cin].t()
-            return wt
-        return m.reshape(Cout, k, k, Cin).permute(0, 3, 1, 2).contiguous()
-
-    class _W:
-        def effective(self_inner):
-            return tuple(None if t is None else unpack(t) for t in wp.effective())
-    exp = F.relu(_expected(x, _W(), lambda xx, ww: _ref_conv(xx, ww, mode, k), P) + bias.view(1, -1, 1, 1))
+    unpack = lambda m: _unpack(m, Cin, Cout, mode, k)
     got = _planes_value(out)
-    # remaining differences: fp32 accumulation order over K (<= 3456 terms), the dropped lo*lo term (P=2), and the
-    # precision of the OUTPUT planes themselves (P=1: 11 bits; P=3: ~15 bits; P=2: ~22 bits)
-    atol, rtol = {2: (1e-4, 0), 3: (1.5e-4, 1e-4), 1: (5e-4, 1.1e-3)}[P]
     np.testing.assert_allclose(got.numpy(), exp.numpy(), atol=atol, rtol=rtol)
     if P != 3:      # both CTA shapes: one or two 128-pixel M tiles per weight tile (K stages of 64 / 32 channels)
         for tm in (1, 2):
@@ -190,72 +201,126 @@ def test_conv_gemm_spade_epilogue(C, P):
     np.testing.assert_allclose(_planes_value(chk).numpy(), exp.numpy(), atol={2: 1e-4, 3: 1.5e-3, 1: 3e-3}[P], rtol=0)
 
 
+def _heads_problem(S, P):
+    """seeded heads operands and the fp32 reference: (x, wi, wm, bgimg, ei, em, tol)"""
+    from ipercore_b200 import ops
+    from ipercore_b200.ops import Planes
+    N = 2
+    x = F.relu(_rand((N, 64, S, S), 31)); wi = _rand((3, 64, 5, 5), 32, 0.03); wm = _rand((1, 64, 5, 5), 33, 0.03)
+    bgimg = _rand((1, 3, S, S), 34)
+    xq = _planes_value(Planes.from_nchw(x.to(DEV), P))
+    q = lambda t: ops.split_planes(t, P).float().sum(0)
+    ei = torch.tanh(F.conv2d(xq, q(wi), padding=2)); em = torch.sigmoid(F.conv2d(xq, q(wm), padding=2))
+    return x, wi, wm, bgimg, ei, em, {2: 3e-5, 3: 3e-4, 1: 2e-3}[P]
+
+
+def _check_heads(img, mask, pred, ei, em, bgimg, tol, label):
+    for name, got, exp, t in (("img", img, ei, tol), ("mask", mask, em, tol), ("pred", pred, em * bgimg + (1 - em) * ei, 1.5 * tol)):
+        got = torch.as_tensor(got).cpu()
+        print("%s %s: max |err| %.2e" % (label, name, float((got - exp).abs().max())))
+        np.testing.assert_allclose(got.numpy(), exp.numpy(), atol=t, rtol=0)
+
+
 @pytest.mark.parametrize("S,P", [(32, 2), (300, 2), (300, 3), (64, 1)])
 def test_conv_gemm_heads_epilogue(S, P):
     """5x5 heads (64->3 tanh, 64->1 sigmoid) + composite (imitator.py:393)."""
     from ipercore_b200 import ops
     from ipercore_b200.ops import Planes
     N = 2
-    x = F.relu(_rand((N, 64, S, S), 31)); wi = _rand((3, 64, 5, 5), 32, 0.03); wm = _rand((1, 64, 5, 5), 33, 0.03)
-    bgimg = _rand((1, 3, S, S), 34)
-    a = Planes.from_nchw(x.to(DEV), P); xq = _planes_value(a)
+    x, wi, wm, bgimg, ei, em, tol = _heads_problem(S, P)
+    a = Planes.from_nchw(x.to(DEV), P)
     wp = ops.pack_heads_weight(wi, wm, P).to(DEV)
     img = torch.empty((N, 3, S, S), device=DEV); mask = torch.empty((N, 1, S, S), device=DEV); pred = torch.empty((N, 3, S, S), device=DEV)
     ops.conv_gemm(a, wp, ops.IPER_CONV_ROW5, 5, 32, 32, ops.IPER_EPI_HEADS, heads=dict(img=img, mask=mask, pred=pred, bg=bgimg.to(DEV)))
-    q = lambda t: ops.split_planes(t, P).float().sum(0)
-    ei = torch.tanh(F.conv2d(xq, q(wi), padding=2)); em = torch.sigmoid(F.conv2d(xq, q(wm), padding=2))
-    tol = {2: 3e-5, 3: 3e-4, 1: 2e-3}[P]
-    np.testing.assert_allclose(img.cpu().numpy(), ei.numpy(), atol=tol, rtol=0)
-    np.testing.assert_allclose(mask.cpu().numpy(), em.numpy(), atol=tol, rtol=0)
-    np.testing.assert_allclose(pred.cpu().numpy(), (em * bgimg + (1 - em) * ei).numpy(), atol=1.5 * tol, rtol=0)
-    if True:        # halo kernel: 32x4 tiles, the five vertical taps are views of one 32x8 box
-        img2 = torch.full_like(img, 9.0); mask2 = torch.full_like(mask, 9.0); pred2 = torch.full_like(pred, 9.0)
-        ops.conv_gemm(a, wp, ops.IPER_CONV_ROW5, 5, 32, 32, ops.IPER_EPI_HEADS,
-                      heads=dict(img=img2, mask=mask2, pred=pred2, bg=bgimg.to(DEV)), cta_pair=2)
-        np.testing.assert_allclose(img2.cpu().numpy(), ei.numpy(), atol=tol, rtol=0)
-        np.testing.assert_allclose(mask2.cpu().numpy(), em.numpy(), atol=tol, rtol=0)
-        np.testing.assert_allclose(pred2.cpu().numpy(), (em * bgimg + (1 - em) * ei).numpy(), atol=1.5 * tol, rtol=0)
-        if P == 2:  # the default above concatenates [w_hi ; w_lo] along N (2 MMAs per K step); the 3-MMA form must agree
-            import os
-            os.environ["IPER_HEADS_CAT"] = "0"
-            try:
-                img3 = torch.full_like(img, 9.0)
-                ops.conv_gemm(a, wp, ops.IPER_CONV_ROW5, 5, 32, 32, ops.IPER_EPI_HEADS, heads=dict(img=img3), cta_pair=2)
-                torch.cuda.synchronize()
-            finally:
-                del os.environ["IPER_HEADS_CAT"]
-            np.testing.assert_allclose(img3.cpu().numpy(), img2.cpu().numpy(), atol=2e-6, rtol=0)
+    _check_heads(img, mask, pred, ei, em, bgimg, tol, "heads S=%d P=%d" % (S, P))
+    # halo kernel: 32x4 tiles, the five vertical taps are views of one 32x8 box (with P=2: the N-concatenated
+    # [w_hi ; w_lo] form, 2 MMAs per K step; the 3-MMA form runs in test_heads_three_mma_form)
+    img2 = torch.full_like(img, 9.0); mask2 = torch.full_like(mask, 9.0); pred2 = torch.full_like(pred, 9.0)
+    ops.conv_gemm(a, wp, ops.IPER_CONV_ROW5, 5, 32, 32, ops.IPER_EPI_HEADS,
+                  heads=dict(img=img2, mask=mask2, pred=pred2, bg=bgimg.to(DEV)), cta_pair=2)
+    _check_heads(img2, mask2, pred2, ei, em, bgimg, tol, "heads halo S=%d P=%d" % (S, P))
 
 
-def test_stem_and_attention_kernels():
+# ----------------------------------------------------------------------------------------------------------------------
+# IPER_HEADS_CAT=0 / IPER_CONVT_FUSE_N=0: read once per process by the library, so they run in one child process
+# ----------------------------------------------------------------------------------------------------------------------
+HEADS_3MMA = [(32, 2), (300, 2)]
+# the mode-2 rows of CASES the halo (cta_pair = 2) kernel takes: the only kernel with fused transposed-conv phases
+CONVT_UNFUSED = [(c, P) for c in CASES if c[5] == 2 and _halo_ok(2, 4, 256 if c[4] >= 256 else c[4], c[1], c[2]) for P in (1, 2)]
+VARIANT_ENV = {"IPER_HEADS_CAT": "0", "IPER_CONVT_FUSE_N": "0"}
+
+
+def child_heads_convt(inputs):
+    """the halo kernel on the HEADS_3MMA and CONVT_UNFUSED problems (this process's switches)"""
     from ipercore_b200 import ops
     from ipercore_b200.ops import Planes
-    import math
+    t = lambda k: torch.from_numpy(inputs[k])
+    out = {}
+    for S, P in HEADS_3MMA:
+        a = Planes.from_nchw(t("h%d_%d_x" % (S, P)).to(DEV), P)
+        wp = ops.pack_heads_weight(t("h%d_%d_wi" % (S, P)), t("h%d_%d_wm" % (S, P)), P).to(DEV)
+        hd = {k: torch.full((2, c, S, S), 9.0, device=DEV) for k, c in (("img", 3), ("mask", 1), ("pred", 3))}
+        ops.conv_gemm(a, wp, ops.IPER_CONV_ROW5, 5, 32, 32, ops.IPER_EPI_HEADS,
+                      heads=dict(hd, bg=t("h%d_%d_bg" % (S, P)).to(DEV)), cta_pair=2)
+        out.update({"h%d_%d_%s" % (S, P, k): v.cpu().numpy() for k, v in hd.items()})
+    for i, ((N, H, W, Cin, Cout, mode, k), P) in enumerate(CONVT_UNFUSED):
+        a = Planes.from_nchw(t("c%d_x" % i).to(DEV), P)
+        wp = ops.pack_convT_weight(t("c%d_w" % i), P).to(DEV)
+        o = Planes.empty(P, N, 2 * H, 2 * W, Cout, DEV)
+        o.data.fill_(7.0)
+        ops.conv_gemm(a, wp, mode, k, Cout, Cout, ops.IPER_EPI_PLANES, bias=t("c%d_b" % i).to(DEV), relu=True, out=o,
+                      cta_pair=2)
+        out["c%d_out" % i] = o.to_nchw().cpu().numpy()
+    torch.cuda.synchronize()
+    return out
+
+
+@pytest.fixture(scope="module")
+def variant_outputs(tmp_path_factory):
+    from test_attention_gpu import run_variant
+    inputs = {}
+    for S, P in HEADS_3MMA:
+        x, wi, wm, bgimg = _heads_problem(S, P)[:4]
+        inputs.update({"h%d_%d_x" % (S, P): x.numpy(), "h%d_%d_wi" % (S, P): wi.numpy(), "h%d_%d_wm" % (S, P): wm.numpy(),
+                       "h%d_%d_bg" % (S, P): bgimg.numpy()})
+    for i, (case, P) in enumerate(CONVT_UNFUSED):
+        x, w, bias = _planes_problem(*case, P)[:3]
+        inputs.update({"c%d_x" % i: x.numpy(), "c%d_w" % i: w.numpy(), "c%d_b" % i: bias.numpy()})
+    out, kernels = run_variant(tmp_path_factory.mktemp("variants"), VARIANT_ENV, "test_conv_gpu", "child_heads_convt", inputs)
+    print("child with %s ran: %s" % (VARIANT_ENV, ", ".join(sorted({n.split("(")[0] for n in kernels}))))
+    return out
+
+
+@pytest.mark.parametrize("S,P", HEADS_3MMA)
+def test_heads_three_mma_form(S, P, variant_outputs):
+    """IPER_HEADS_CAT=0: the halo heads kernel with three MMAs per K step (hi*w_hi, hi*w_lo, lo*w_hi) instead of the
+    N-concatenated weights, against the same reference and tolerance as the default form"""
+    x, wi, wm, bgimg, ei, em, tol = _heads_problem(S, P)
+    g = lambda k: torch.from_numpy(variant_outputs["h%d_%d_%s" % (S, P, k)])
+    _check_heads(g("img"), g("mask"), g("pred"), ei, em, bgimg, tol, "heads 3-MMA (IPER_HEADS_CAT=0) S=%d P=%d" % (S, P))
+
+
+@pytest.mark.parametrize("case,P", CONVT_UNFUSED, ids=lambda v: str(v))
+def test_convT_unfused_phases(case, P, variant_outputs):
+    """IPER_CONVT_FUSE_N=0: the halo kernel's transposed convolution with one MMA group per phase, against the
+    reference test_conv_gemm_planes uses"""
+    i = CONVT_UNFUSED.index((case, P))
+    exp, atol, rtol = _planes_problem(*case, P)[3:]
+    got = variant_outputs["c%d_out" % i]
+    print("convT unfused %s P=%d: max |err| %.2e" % (case, P, float(np.abs(got - exp.numpy()).max())))
+    np.testing.assert_allclose(got, exp.numpy(), atol=atol, rtol=rtol)
+
+
+def test_stem_direct_kernel():
+    """the CUDA-core stem (IPER_STEM=direct); iper_warp_attention is tested in test_attention_gpu.py"""
+    from ipercore_b200 import ops
+    from ipercore_b200.ops import Planes
     P, N, S = 2, 2, 64
     x = _rand((N, 6, S, S), 41); w = _rand((64, 6, 3, 3), 42, 0.2); b = _rand((64,), 43, 0.1)
     out = Planes.empty(P, N, S // 2, S // 2, 64, DEV)
     ops.conv_stem(x.to(DEV), w.to(DEV), b.to(DEV), out)
     exp = F.relu(F.conv2d(x, w, b, stride=2, padding=1))
     np.testing.assert_allclose(_planes_value(out).numpy(), exp.numpy(), atol=1e-5, rtol=0)
-    # attention with the projections hoisted to the source side, against the reference formulation
-    # (warp first, then fk/fv/fq 1x1 convs, softmax over sources — attlwb_spade_resunet.py:208-252)
-    for (B, ns, h, C) in ((2, 2, 16, 64), (1, 3, 8, 256)):
-        src = _rand((ns, C, h, h), 44); xt = _rand((B, C, h, h), 45)
-        wq = _rand((C, C, 1, 1), 51, 0.1); bq = _rand((C,), 52, 0.3)
-        wk = _rand((C, C, 1, 1), 46, 0.2); wv = _rand((C, C, 1, 1), 47, 0.2); bk = _rand((C,), 48, 0.3); bv = _rand((C,), 49, 0.1)
-        T = _rand((B, ns, h, h, 2), 50, 1.3)                      # some samples fall outside [-1,1] -> zero padding
-        kv = F.conv2d(src, ops.attention_source_weight(wq, bq, wk, wv)).permute(0, 2, 3, 1).contiguous()
-        xp = Planes.from_nchw(xt.to(DEV), P); xq = _planes_value(xp)
-        att = Planes.empty(P, B, h, h, C, DEV)
-        ops.warp_attention(xp, kv.to(DEV), bv.to(DEV), T.to(DEV), att)
-        exp = []
-        for bi in range(B):
-            warp = F.grid_sample(src, T[bi], mode="bilinear", padding_mode="zeros", align_corners=False)
-            K = F.conv2d(warp, wk, bk); V = F.conv2d(warp, wv, bv)
-            q = F.conv2d(xq[bi:bi + 1], wq, bq)
-            logit = (K * q).sum(1, keepdim=True) / math.sqrt(C)
-            exp.append((torch.softmax(logit, 0) * V).sum(0))
-        np.testing.assert_allclose(_planes_value(att).numpy(), torch.stack(exp).numpy(), atol=3e-5, rtol=0)
 
 
 @pytest.mark.parametrize("N,H,W,Cin,Cout,mode", [(3, 16, 16, 64, 128, 0), (2, 32, 32, 64, 128, 1), (5, 4, 4, 128, 256, 0)])

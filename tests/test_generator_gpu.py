@@ -23,7 +23,10 @@ def _gen(precision):
 
 
 @pytest.mark.parametrize("S,precision,tol", [(256, "fp16x2", 1e-3), (64, "fp16x2", 1e-3), (256, "fp16f8", 1e-3),
-                                             (64, "fp16f8", 1e-3), (256, "fp16", 1e-2)])
+                                             (64, "fp16f8", 1e-3), (256, "fp16", 1e-2),
+                                             # single-plane SPADE convolutions: 6.6e-4 .. 1.8e-3 in the CPU emulation
+                                             # (tools/precision_plan.py); not a 1e-3 mode
+                                             (256, "mixed", 3e-3)])
 def test_forward_src_tsf_matches_reference(S, precision, tol, golden_dir):
     import make_golden
     g = np.load(os.path.join(golden_dir, "gen_S%d.npz" % S))
